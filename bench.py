@@ -2,6 +2,7 @@
 """bench.py -- training throughput of the MicroDiT hot path on B200 (contract: see README / task statement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c3|c4|c5|tiny]
+                    [--dump-outputs DIR]
 
 One "step" = one optimisation step at global batch 2048 (BASELINE.json metric): every rank runs its
 2048/N images as microbatches through LatentDiffusion.forward + backward (the CUDA path through the C ABI),
@@ -11,6 +12,14 @@ batch contract (fp16 latents / fp16 77x1024 captions / caption-drop mask), rando
 `value`  : img/s with the step's inputs already resident in HBM (device-timed, max over ranks).
 `e2e`    : the same through the public API from PINNED HOST buffers, H2D copies and the loss read-back inside
            the timed region.
+`--dump-outputs DIR` : after the timed steps, what the last of them handed its caller, as DIR/<name>.npy (float32):
+           `loss` (the step's mean loss), `params` (updated fp32 parameters) and `adamw_m` (AdamW's first moment, the
+           running mean of the clipped gradient), the latter two at DUMP_SAMPLE fixed seeded positions of the flat
+           buffers.  Weights, batch and the EDM / mask draws are seeded, and the run uses the library's deterministic
+           mode (DESIGN.md section 5.4; `config.deterministic` in the line): the fast path's cross-block float atomics
+           make the gradients differ in the last bits from run to run, and AdamW and the following steps amplify that
+           far beyond rounding.  With fixed-order sums the outputs are a function of the arguments alone, so two runs
+           agree bit for bit and two builds can be compared output for output.
 `--impl reference` : the reference algorithm on the host CPU cores (oracle.port -- the reference itself is pure
            Python/torch and /root/reference does not exist on the GPU box), bounded sample per step.
 """
@@ -24,6 +33,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -133,6 +143,20 @@ def synth_host_batch(B, wl, seed, pinned):
     return b
 
 
+DUMP_SAMPLE = 1 << 22  # entries kept of each flat buffer by --dump-outputs: 16 MiB of float32 each
+
+
+def timed_outputs(ld, opt, loss):
+    """The arrays of --dump-outputs (see the module docstring), on the host."""
+    flat = ld.dit.store.flat
+    idx = None
+    if flat.numel() > DUMP_SAMPLE:
+        g = torch.Generator().manual_seed(1234)
+        idx = torch.randint(flat.numel(), (DUMP_SAMPLE,), generator=g).sort().values.to(flat.device)
+    pick = lambda t: (t if idx is None else t[idx]).float().cpu().numpy()  # noqa: E731
+    return {"loss": loss.float().reshape(1).cpu().numpy(), "params": pick(flat), "adamw_m": pick(opt.m)}
+
+
 def randomize_weights(dit, seed):
     """De-degenerate the zero-initialised tensors (dit.py:615-627) so every block carries signal."""
     g = torch.Generator(device=dit.store.device).manual_seed(seed)
@@ -167,7 +191,7 @@ def host_threads():
 
 def cpu_reference_img_per_s(wl, batch, iters, threads, state_dict=None, budget_s=60.0, warmup=0):
     """The reference algorithm (oracle.port, fp32) forward+backward on the host cores.
-    Runs `warmup` untimed passes, then up to `iters` timed passes, stopping early once `budget_s` is spent.
+    Runs `warmup` untimed passes, then up to `iters` timed passes, stopping early once `budget_s` is spent (None: all).
     Returns (img/s, timed passes done)."""
     from oracle import port, weights
     torch.set_num_threads(threads)
@@ -206,7 +230,7 @@ def cpu_reference_img_per_s(wl, batch, iters, threads, state_dict=None, budget_s
         dt = time.perf_counter() - t0
         if it >= warmup:
             times.append(dt)
-        if time.perf_counter() - t_start > budget_s and times:
+        if budget_s is not None and time.perf_counter() - t_start > budget_s and times:
             break
     return batch * len(times) / sum(times), len(times)
 
@@ -220,16 +244,14 @@ def run_reference_arm(args, wl):
     threads = host_threads()
     sample = 8 if wl["res"] == 32 else 2
     t0 = time.perf_counter()
-    ips, done = cpu_reference_img_per_s(wl, sample, max(1, args.steps), threads, budget_s=150.0,
-                                        warmup=1 if args.warmup > 0 else 0)
+    ips, done = cpu_reference_img_per_s(wl, sample, args.steps, threads, budget_s=None, warmup=1 if args.warmup > 0 else 0)
     wall = time.perf_counter() - t0
     line = {
         "impl": "reference", "metric": "training images/sec (global batch 2048)", "value": ips, "unit": "img/s",
         "n_gpus": args.gpus, "steps": done, "warmup": 1 if args.warmup > 0 else 0, "ms_per_step": 1000.0 * sample / ips,
         "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": wl["name"], "global_batch": GLOBAL_BATCH,
-                   "sample": f"{sample} images per step (forward+backward), {done} of {args.steps} requested steps "
-                             f"inside the 150 s budget"},
+                   "sample": f"{sample} images per step (forward+backward)"},
         "cpu_baseline": {"value": ips, "unit": "img/s", "cores": threads, "kind": "port",
                          "sample": f"{sample}-image forward+backward x {done}, fp32, oracle.port, {threads} threads"},
         "e2e": {"value": ips, "unit": "img/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -252,7 +274,13 @@ def main():
     ap.add_argument("--profile-out", default="")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the brief c3/c4/c5 legs of the N=1 run")
     ap.add_argument("--no-stock-torch", action="store_true", help="skip the stock-PyTorch-on-B200 comparator leg")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the last timed step's loss, parameters and AdamW first moment as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the B200 path")
     wl = dict(WORKLOADS[args.workload])
     if args.impl == "reference":
         run_reference_arm(args, wl)
@@ -271,17 +299,22 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=device)
     assert world == args.gpus or world == 1, "launch with torchrun --nproc-per-node == --gpus"
-    W, K = max(3, args.warmup), max(1, args.steps)
+    W, K = max(3, args.warmup), args.steps
     per_rank = args.global_batch // world
     micro = min(args.microbatch or wl["micro"], per_rank)
 
-    def measure(wl, micro, K, W, with_e2e=True, with_probe=True):
+    def measure(wl, micro, K, W, with_e2e=True, with_probe=True, with_outputs=False):
         """Build the model of workload `wl`, run W warm-up + K timed steps (inputs resident), optionally the end-to-end
-        pass from pinned host memory and the per-launch roofline probe; returns a dict of raw numbers and frees the model."""
+        pass from pinned host memory and the per-launch roofline probe; returns a dict of raw numbers and frees the model.
+        `with_outputs`: also the host copies of what the last timed step returned (timed_outputs)."""
+        torch.manual_seed(18)  # weight init and the EDM / mask draws of every step
         ld = build_model(wl, device)
         opt = FlatAdamW(ld.dit, lr=2.4e-4, weight_decay=0.1, clip_norm=0.25)
         reducer = GradReducer(ld.dit.store, ops=ld.dit.engine.ops) if world > 1 else None
         ops = ld.dit.engine.ops
+        deterministic = with_outputs or os.environ.get("MD_DETERMINISTIC", "0") == "1"
+        if with_outputs:
+            ops.set_deterministic(True)
 
         host = synth_host_batch(per_rank, wl, seed=18 + rank, pinned=True)
         h2d_bytes = sum(v.numel() * v.element_size() for v in host.values())
@@ -333,7 +366,11 @@ def main():
         value = args.global_batch / (ms_step / 1e3)
 
         r = dict(value=value, ms_step=ms_step, launches=launches, clocks=clocks, loss=float(loss_t), micro=micro,
-                 h2d_bytes=h2d_bytes, step_tflops=(value / world) * wl["gf"] / 1e3 if wl["gf"] else None)
+                 h2d_bytes=h2d_bytes, step_tflops=(value / world) * wl["gf"] / 1e3 if wl["gf"] else None,
+                 deterministic=deterministic)
+        if with_outputs:
+            opt.gather_state()  # sharded optimizer: complete the moments (a collective: every rank calls it)
+            r["outputs"] = timed_outputs(ld, opt, loss_t) if rank == 0 else None
         # ---- end to end from pinned host memory
         if with_e2e:
             step_e2e()
@@ -374,6 +411,8 @@ def main():
                 "NCCL all-reduce (mean) of the flat fp32 gradient, replicated clip + AdamW") + \
                 f"; overlap with backward={reducer.overlap}, {reducer.reserve} SMs left to NCCL while it overlaps"
         r["peak_hbm_gb"] = torch.cuda.max_memory_allocated(device) / 2 ** 30
+        if deterministic and os.environ.get("MD_DETERMINISTIC", "0") != "1":
+            ops.set_deterministic(False)  # process-wide switch: the other workloads' legs run the fast path
         r["state_dict"] = ({k: v.detach().cpu() for k, v in ld.dit.state_dict().items()}
                            if (rank == 0 and with_probe and not args.no_cpu_baseline and world == 1) else None)
         del ld, opt, ops, resident, host, reducer, step_resident, step_e2e
@@ -384,7 +423,7 @@ def main():
         return r
 
     peaks = read_peaks()
-    m = measure(wl, micro, K, W)
+    m = measure(wl, micro, K, W, with_outputs=bool(args.dump_outputs))
     value, ms_step, launches, clocks = m["value"], m["ms_step"], m["launches"], m["clocks"]
     prof, tot_ms, gemm_ms, gemm_n, gemm_tflops, step_tflops = (m["prof"], m["tot_ms"], m["gemm_ms"], m["gemm_n"],
                                                                m["gemm_tflops"], m["step_tflops"])
@@ -425,6 +464,10 @@ def main():
                         continue
                     tf = f"{fl / (ms * 1e-3) / 1e12:.1f}" if fl else ""
                     f.write(f"{k},{n},{ms:.3f},{ms / tot_ms:.4f},{tf}\n")
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in m["outputs"].items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         cpu_base = None
         if not args.no_cpu_baseline and world == 1:
             threads = host_threads()
@@ -440,7 +483,8 @@ def main():
             "steps": K, "warmup": W, "ms_per_step": ms_step, "higher_is_better": True, "scaling": "strong",
             "vs_baseline": None, "dtype": "bf16", "data": "synthetic",
             "config": {"workload": wl["name"], "global_batch": args.global_batch, "per_gpu_batch": per_rank,
-                       "microbatch": micro, "parallelism": f"dp{world}", "optimizer": "clip0.25+AdamW (fused, in step)",
+                       "microbatch": micro, "parallelism": f"dp{world}", "deterministic": m["deterministic"],
+                       "optimizer": "clip0.25+AdamW (fused, in step)",
                        "l2": "per-step working set (activations > 40 GB per microbatch) far exceeds the 126 MB L2",
                        "grad_exchange": m["grad_exchange"]},
             "e2e": {"value": e2e_value, "unit": "img/s", "ms_per_step": ms_e2e, "h2d_bytes_per_step": h2d_bytes,

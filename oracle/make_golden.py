@@ -1,6 +1,8 @@
-"""Generate tests/golden/parity_<cfg>.pt from the UNMODIFIED reference (dev container only).
+"""Generate the fixtures under tests/golden/ from the UNMODIFIED reference (needs its source tree, see oracle.ref_import).
 
-    python -m oracle.make_golden
+    python -m oracle.make_golden             # parity_<cfg>.pt
+    python -m oracle.make_golden sampler     # sampler_<cfg>.pt
+    python -m oracle.make_golden reference   # reference_grads_<cfg>.pt, reference_get_mask.pt, reference_configs/
 
 For every config in oracle.configs.PARITY_CONFIGS: synthetic non-degenerate weights (oracle.weights, seed 7),
 synthetic batch (seed 11), the reference's three random draws replayed from torch.manual_seed(123)
@@ -15,6 +17,7 @@ from __future__ import annotations
 
 import os
 import sys
+import zlib
 
 import torch
 
@@ -33,17 +36,24 @@ def fingerprint(name, g):
     return float(g.norm()), float((g * pr).sum())
 
 
+def reference_case(ref_dit, c):
+    """The reference DiT of config `c` with the seeded weights, its LatentDiffusion (train mode) and the seeded batch."""
+    ct = c["ctor"]
+    net = ref_dit.DiT(**ct)
+    sd = weights.synth_state_dict(net.state_dict(), seed=WEIGHT_SEED)
+    net.load_state_dict(sd)
+    ld = ref_import.build_reference_latent_diffusion(net, c["p_mean"], c["p_std"], c["mask_ratio"], ct["input_size"])
+    ld.train()
+    batch = weights.synth_batch(c["batch"], ct["in_channels"], ct["input_size"], seed=BATCH_SEED)
+    return net, sd, ld, batch
+
+
 def main():
     ref_dit, ref_model, _ = ref_import.load_reference()
     out_dir = os.path.join(ROOT, "tests", "golden")
     for name, c in configs.PARITY_CONFIGS.items():
         ct = c["ctor"]
-        net = ref_dit.DiT(**ct)
-        sd = weights.synth_state_dict(net.state_dict(), seed=WEIGHT_SEED)
-        net.load_state_dict(sd)
-        ld = ref_import.build_reference_latent_diffusion(net, c["p_mean"], c["p_std"], c["mask_ratio"], ct["input_size"])
-        ld.train()
-        batch = weights.synth_batch(c["batch"], ct["in_channels"], ct["input_size"], seed=BATCH_SEED)
+        net, sd, ld, batch = reference_case(ref_dit, c)
         res = {}
         for mode in ("fp32", "bf16"):
             net.zero_grad()
@@ -120,8 +130,63 @@ def main_sampler(names=("P", "S")):
         print(name, {k: (tuple(v.shape), float(v.abs().mean())) for k, v in fx.items() if torch.is_tensor(v)})
 
 
+GRAD_SAMPLE, GRAD_SAMPLE_SEED = 128, 41
+
+
+def grad_sample_index(key, numel):
+    """Flat indices of the gradient entries of parameter `key` kept in reference_grads_<cfg>.pt: all of them up to
+    GRAD_SAMPLE, else a fixed sample drawn from a generator seeded by the key."""
+    if numel <= GRAD_SAMPLE:
+        return torch.arange(numel)
+    g = torch.Generator().manual_seed((GRAD_SAMPLE_SEED * 1000003 + zlib.crc32(key.encode())) % (2 ** 31 - 1))
+    return torch.randperm(numel, generator=g)[:GRAD_SAMPLE]
+
+
+def main_reference_grads():
+    """tests/golden/reference_grads_<cfg>.pt: the reference's fp32 loss and, for every parameter in `names` order, its
+    gradient at the entries grad_sample_index() picks, concatenated -- the same case as main()."""
+    ref_dit, _, _ = ref_import.load_reference()
+    out_dir = os.path.join(ROOT, "tests", "golden")
+    for name, c in configs.PARITY_CONFIGS.items():
+        net, _, ld, batch = reference_case(ref_dit, c)
+        torch.manual_seed(DRAW_SEED)
+        loss, _, _ = ld({k: v.clone() for k, v in batch.items()})
+        loss.backward()
+        names = [k for k, _ in net.named_parameters()]
+        sample = torch.cat([p.grad.detach().reshape(-1)[grad_sample_index(k, p.numel())] for k, p in net.named_parameters()])
+        path = os.path.join(out_dir, f"reference_grads_{name}.pt")
+        torch.save({"config": name, "loss": loss.item(), "names": names, "grad_sample": sample,
+                    "torch_version": torch.__version__}, path)
+        print(f"{name}: loss {loss.item():.7f}, {len(names)} gradients -> {path} ({os.path.getsize(path) / 1024:.0f} KiB)")
+
+
+def main_reference_mask():
+    """tests/golden/reference_get_mask.pt: get_mask (utils.py:383-399) of the reference after torch.manual_seed(5)."""
+    _, _, ref_utils = ref_import.load_reference()
+    torch.manual_seed(5)
+    m = ref_utils.get_mask(3, 64, 0.75, torch.device("cpu"))
+    torch.save({k: m[k].clone() for k in ("ids_keep", "ids_restore", "mask")},
+               os.path.join(ROOT, "tests", "golden", "reference_get_mask.pt"))
+
+
+def main_reference_configs():
+    """tests/golden/reference_configs/: the reference's training YAML files, byte for byte."""
+    import shutil
+    src = os.path.join(ref_import.REFERENCE_ROOT, "configs")
+    dst = os.path.join(ROOT, "tests", "golden", "reference_configs")
+    os.makedirs(dst, exist_ok=True)
+    for f in sorted(os.listdir(src)):
+        if f.endswith(".yaml"):
+            shutil.copyfile(os.path.join(src, f), os.path.join(dst, f))
+            print(f"{f} -> {dst}")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "sampler":
         main_sampler()
+    elif len(sys.argv) > 1 and sys.argv[1] == "reference":
+        main_reference_grads()
+        main_reference_mask()
+        main_reference_configs()
     else:
         main()

@@ -7,8 +7,8 @@ and derives the architecture from the tensor shapes.  Each function cites the re
 the unmodified reference can be replayed draw for draw (SURVEY.md section 3.2: sigma-normal -> eps ->
 mask noise).
 
-Pinned against the live reference by tests/test_oracle_pinned.py (dev container) and against the
-committed fixtures tests/golden/*.pt everywhere.
+Pinned against the reference by tests/test_oracle_pinned.py through the committed fixtures tests/golden/*.pt,
+generated from the reference by oracle/make_golden.py.
 """
 from __future__ import annotations
 

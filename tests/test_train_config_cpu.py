@@ -7,7 +7,8 @@ import yaml
 
 from tests import parity_common as pc
 
-REF_CONFIGS = "/root/reference/configs"
+# the reference's configs/*.yaml, stored unchanged (oracle/make_golden.py reference)
+REF_CONFIGS = os.path.join(pc.GOLDEN, "reference_configs")
 
 MINI = """
 exp_name: mini_run
@@ -90,7 +91,6 @@ def test_interpolation_overrides_and_trainer_kwargs(tmp_path):
         train.apply_overrides({}, ["novalue"])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CONFIGS), reason="reference configs only exist in the dev container")
 @pytest.mark.parametrize("name", ["res_256_pretrain", "res_256_finetune", "res_512_pretrain", "res_512_finetune"])
 def test_every_reference_yaml_maps_onto_the_trainer(name):
     from micro_diffusion_b200 import train
